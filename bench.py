@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- particle-steps/sec of the SMC hot path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (config 2 of BASELINE.json): bootstrap filter of the stochastic-volatility
 model (StochVol defaults), N = 1e7 particles per GPU, systematic resampling,
@@ -31,11 +31,13 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True     # the tree may be read-only: no __pycache__ next to the sources
 
 N_PER_GPU = 10_000_000
 ESSRMIN = 0.5
 SCHEME = "systematic"
 HBM_FALLBACK_GBS = 6650.0      # B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
+DUMP_SAMPLE = 1 << 19          # particles (and summary rows) written by --dump-outputs
 FP64_INST_PER_PAIR = 105       # fp64 instructions of the streaming step per pair of particles; superseded by the
                                # committed ncu capture (profiles/*_ncu_summary.json: move.fp64_inst_per_pair) when present
 
@@ -228,7 +230,7 @@ def run_reference(args):
     # workers 2.2e8, 32 workers 1.5e8, 128 workers 0.9e8 particle-steps/s in aggregate): capped at 16
     workers = max(1, min(cores, mem_workers, 16))
     n = N_PER_GPU
-    K = max(1, min(args.steps, 4))              # bounded sample: ~3 s per step per worker
+    K = args.steps
     reps = max(1, min(args.warmup, 1))
     live = have_live_reference()
     for _ in range(reps):
@@ -320,6 +322,28 @@ def workload(args, K):
         ssm=kalman.MVLinearGauss_Guarniero_etal(alpha=0.4, dx=4), data=yl), y, "stratified", ESSRMIN, 4, False)
 
 
+def dump_outputs(path, eng, table):
+    """--dump-outputs: what a caller of the timed filter receives after its last step, as float64 .npy files:
+    X (particles, (N,) or (N, d)), lw (log-weights), A (ancestors; the identity when that step did not resample, and
+    so after a single step, where the public API's SMC.A is None) and the per-step ESSs / logLts / rs_flags.  Of more than DUMP_SAMPLE particles a fixed seeded sample is written (its
+    indices in index.npy), of more than DUMP_SAMPLE steps the last ones: at most (d + 3) * 4 MB + 12 MB in all."""
+    import torch
+    cur = (table.shape[0] - 1) & 1                 # step s writes buffers [s & 1]
+    idx = np.arange(eng.N)
+    if eng.N > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(0).choice(eng.N, DUMP_SAMPLE, replace=False))
+    sel = torch.from_numpy(idx).to(eng.A.device)
+    x = eng.X[cur].index_select(eng.X[cur].ndim - 1, sel)
+    rows = table[-DUMP_SAMPLE:]
+    out = {"index": idx, "X": x.t() if x.ndim > 1 else x, "lw": eng.lw[cur].index_select(0, sel),
+           "A": eng.A.index_select(0, sel) if table[-1, 2] else sel,
+           "ESSs": rows[:, 0], "logLts": rows[:, 1], "rs_flags": rows[:, 2]}
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        a = a.cpu().numpy() if isinstance(a, torch.Tensor) else a
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -385,6 +409,8 @@ def run_b200(args):
     table = eng.summ.cpu().numpy()
     n_rs = int(table[:, 2].sum())
     logLt = float(table[K - 1, 1])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, table)
     eng.close()
 
     # per-kernel CUDA-event timing of the same K steps (separate pass, same kernels)
@@ -535,7 +561,9 @@ def run_b200(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=int, default=None,
+                    help="timed filter steps (default: 1000 for c2, 500 for c3i / c3ii; 4 with --impl reference, "
+                         "about 3 s per step per worker)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--n", type=int, default=None, help="particles per GPU (default: 1e7 for c2, 1e6 for c3)")
@@ -548,13 +576,21 @@ def main():
                          "resampling with ancestors pulled over NVLink")
     ap.add_argument("--essrmin", type=float, default=0.5,
                     help="0.5 = BASELINE config 2; 1.0 = resample at every step (stress case)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps write what the timed filter computed in its last step to DIR/*.npy "
+                         "(float64; more than %d particles: a fixed seeded sample; rank 0's shard on N > 1 GPUs)"
+                         % DUMP_SAMPLE)
     args = ap.parse_args()
     global ESSRMIN
     ESSRMIN = args.essrmin
     if args.n is None:
         args.n = N_PER_GPU if args.config == "c2" else 1_000_000
-    if args.config != "c2" and args.steps == 1000:
-        args.steps = 500
+    if args.steps is None:
+        args.steps = 4 if args.impl == "reference" else 1000 if args.config == "c2" else 500
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the GPU filter (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -10,8 +10,10 @@ set -e
 cd "$(dirname "$0")"
 SRC=${1:-/root/reference}
 if [ ! -d "$SRC/particles" ]; then echo "no reference at $SRC: oracle/_ref left as it is"; exit 0; fi
+# a read-only reference checkout must not give a read-only copy: the next line, and the next build, delete in it
+if [ -d _ref ]; then chmod -R u+w _ref; fi
 rm -rf _ref && mkdir -p _ref
-cp -r "$SRC/particles" _ref/particles
+cp -r --no-preserve=mode "$SRC/particles" _ref/particles
 rm -rf _ref/particles/datasets _ref/particles/__pycache__        # 3 MB of data files the hot path never reads
 cp "$SRC/LICENSE" _ref/LICENSE 2>/dev/null || true
 echo "oracle/_ref/particles: $(find _ref -name '*.py' | wc -l) modules"

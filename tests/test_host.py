@@ -4,6 +4,7 @@ restatement used by the GPU tests, and the no-CPU-fallback rule.  No compute cal
 import ctypes
 import os
 import re
+import shutil
 import subprocess
 import sys
 
@@ -41,8 +42,11 @@ def test_library_exports_every_declared_symbol(lib):
 
 
 def test_built_for_sm_100a_only():
-    from particles_b200 import _lib
-    out = subprocess.run(["cuobjdump", "-lelf", _lib.SO_PATH], capture_output=True, text=True).stdout
+    from particles_b200 import _lib, build
+    nvcc = shutil.which(build._nvcc())
+    assert nvcc, f"{build._nvcc()} not found: the CUDA toolkit that built the library is needed to inspect it"
+    cuobjdump = os.path.join(os.path.dirname(nvcc), "cuobjdump")   # from the toolkit that built the library
+    out = subprocess.run([cuobjdump, "-lelf", _lib.SO_PATH], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_(\d+a?)", out))
     assert archs == {"100a"}, archs
 
@@ -107,29 +111,42 @@ def test_fused_spec_recognition():
         ssm.fused_spec(ssm.Bootstrap(ssm=ssm.StochVol(), data=[np.zeros(2)] * 3))
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/particles"), reason="reference not mounted")
+def _reference_model(g, name):
+    """A model object as the reference builds it: class name, module and instance attributes recorded from the
+    reference in tests/golden/golden_dropin.npz (make_golden_dropin.py)."""
+    cls = type(name, (), {"__module__": str(g[f"model/{name}/module"])})
+    obj = cls()
+    prefix = f"model/{name}/attr/"
+    for key in g.files:
+        if key.startswith(prefix):
+            v = g[key]
+            setattr(obj, key[len(prefix):], v.item() if v.ndim == 0 else v)
+    return obj
+
+
+def _reference_fk(g, name, ssm, data):
+    """A Feynman-Kac object of the reference's class ``name``: same class names along the method resolution order."""
+    base = None
+    for nm in reversed([str(s) for s in g[f"fk/{name}/mro"]]):
+        base = type(nm, () if base is None else (base,), {})
+    fk = base()
+    fk.ssm, fk.data, fk.T = ssm, data, len(data)
+    return fk
+
+
 def test_reference_objects_are_recognised():
     """Drop-in: a Feynman-Kac object built from the REFERENCE's own classes maps onto the
-    same fused kernel constants as ours (build container only)."""
-    code = r'''
-import sys, numpy as np
-sys.path.insert(0, "/root/reference"); sys.path.insert(0, %r)
-import particles
-from particles import state_space_models as rssm, kalman as rk
-from particles_b200 import state_space_models as ssm, kalman
-y = [np.array([0.3 * i]) for i in range(5)]
-for ref, ours in [(rssm.StochVol(mu=-0.5), ssm.StochVol(mu=-0.5)),
-                  (rk.LinearGauss(rho=0.7), kalman.LinearGauss(rho=0.7)),
-                  (rssm.Gordon_etal(), ssm.Gordon_etal()), (rssm.ThetaLogistic(), ssm.ThetaLogistic())]:
-    a = ssm.fused_spec(rssm.Bootstrap(ssm=ref, data=y)); b = ssm.fused_spec(ssm.Bootstrap(ssm=ours, data=y))
-    assert a["model"] == b["model"] and a["fk"] == b["fk"] and list(a["params"]) == list(b["params"])
-    assert np.array_equal(a["data"], b["data"])
-assert ssm.fused_spec(rssm.AuxiliaryPF(ssm=rssm.StochVol(), data=y))["fk"] == 2
-print("ok")
-''' % ROOT
-    env = dict(os.environ, PYTHONDONTWRITEBYTECODE="1")
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env)
-    assert r.stdout.strip().endswith("ok"), r.stderr[-2000:]
+    same fused kernel constants as ours."""
+    from particles_b200 import kalman, state_space_models as ssm
+    g = np.load(os.path.join(ROOT, "tests", "golden", "golden_dropin.npz"))
+    y = [np.array([0.3 * i]) for i in range(5)]
+    for name, ours in [("StochVol", ssm.StochVol(mu=-0.5)), ("LinearGauss", kalman.LinearGauss(rho=0.7)),
+                       ("Gordon_etal", ssm.Gordon_etal()), ("ThetaLogistic", ssm.ThetaLogistic())]:
+        a = ssm.fused_spec(_reference_fk(g, "Bootstrap", _reference_model(g, name), y))
+        b = ssm.fused_spec(ssm.Bootstrap(ssm=ours, data=y))
+        assert a["model"] == b["model"] and a["fk"] == b["fk"] and list(a["params"]) == list(b["params"])
+        assert np.array_equal(a["data"], b["data"])
+    assert ssm.fused_spec(_reference_fk(g, "AuxiliaryPF", _reference_model(g, "StochVol"), y))["fk"] == 2
 
 
 def test_no_cpu_fallback():
